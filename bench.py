@@ -6,7 +6,7 @@ Workload (BASELINE.json configs[2], the configuration the metric is quoted on):
     hnsw(m=32, efconstruction=200, efsearch=64); a *step* = one batch of `--batch` k-NN queries
     (k = efsearch = 64) through the search path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Our arm     : the CUDA path.  `value` = queries/s with the query batch already resident in HBM
               (pgemb_search_batch_device on torch's stream, CUDA-event timed, max over ranks);
@@ -64,7 +64,8 @@ def log(*a):
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=30)
+    ap.add_argument("--steps", type=int, default=30, help="timed steps of the headline search (and of its e2e loop); the legs "
+                    "for the other configurations use their own step counts, which each reports in its JSON")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--rows", dest="n", type=int, default=int(os.environ.get("PGEMB_BENCH_N", 1_000_000)),
@@ -74,7 +75,33 @@ def parse():
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="target CPU time of the cpu_baseline sample")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg (development)")
     ap.add_argument("--no-legs", action="store_true", help="headline only: skip the configs1 / scan_topk / sharded legs (development)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned (labels, counts, counters) "
+                    "as DIR/<name>.npy, so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the CUDA path's results; the reference arm has none to write")
+    return args
+
+
+DUMP_LIMIT = 64 << 20     # bytes --dump-outputs writes at most
+
+
+def dump_outputs(out_dir, labels, n, stats):
+    """The last timed step's results as float64 .npy files: labels [B, k] (unused tail -1), n [B], stats [B, 4], and the
+    queries they belong to (query_index [B]).  A batch too large for DUMP_LIMIT is cut to a fixed, seeded sample of queries."""
+    arrays = {"labels": labels, "n": n, "stats": stats}
+    B = labels.shape[0]
+    per_query = 8 * (sum(a[0].size for a in arrays.values()) + 1)
+    rows = np.arange(B)
+    if B * per_query > DUMP_LIMIT - 4096:          # room for the four .npy headers
+        rows = np.sort(np.random.default_rng(0).choice(B, (DUMP_LIMIT - 4096) // per_query, replace=False))
+    arrays = {name: a[rows] for name, a in arrays.items()}
+    arrays["query_index"] = rows
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.astype(np.float64))
 
 
 # ---------------------------------------------------------------------------------------------------
@@ -281,6 +308,8 @@ def main():
     ms = ev0.elapsed_time(ev1)
     launches = int(lib.pgemb_launch_count()) - launches0
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, d_lab.cpu().numpy(), d_nres[K - 1].cpu().numpy(), d_stats[K - 1].cpu().numpy())
     tms = torch.tensor([ms], device="cuda")
     if world > 1:
         dist.all_reduce(tms, op=dist.ReduceOp.MAX)

@@ -2,6 +2,7 @@
 include/pgemb_b200.h declares, HnswMetadata has the reference's layout, and the product path fails
 loudly (no fallback) when no CUDA device is usable."""
 import ctypes as C
+import json
 import os
 import re
 
@@ -35,10 +36,17 @@ def test_metadata_layout_matches_reference(lib):
     # embedding.h:28-42: 10 size_t + idx_t + enum
     assert C.sizeof(HnswMetadata) == 10 * 8 + 4 + 4
     assert HnswMetadata.enterpoint_node.offset == 80 and HnswMetadata.dist_func.offset == 84
-    ref_h = "/root/reference/embedding.h"
-    if os.path.isfile(ref_h):
-        ref_fields = re.findall(r"^\s*(?:size_t|idx_t|dist_func_t)\s+(\w+);", open(ref_h).read(), re.M)
-        assert ref_fields == [f[0] for f in HnswMetadata._fields_]
+    fields = [f[0] for f in HnswMetadata._fields_]
+    # the reference's field names, as stored from its embedding.h by tests/golden/gen_ref_outputs.py
+    assert fields == json.load(open(os.path.join(ROOT, "tests", "golden", "ref_outputs.json")))["metadata_fields"]
+    ref_dir = os.environ.get("PGEMB_REFERENCE_DIR")
+    if ref_dir and os.path.isfile(os.path.join(ref_dir, "embedding.h")):   # and the reference tree itself where it is present
+        assert reference_metadata_fields(os.path.join(ref_dir, "embedding.h")) == fields
+
+
+def reference_metadata_fields(embedding_h):
+    """HnswMetadata's field names in the reference's embedding.h, in declaration order."""
+    return re.findall(r"^\s*(?:size_t|idx_t|dist_func_t)\s+(\w+);", open(embedding_h).read(), re.M)
 
 
 def test_meta_init_follows_hnsw_get_index(lib):
@@ -162,11 +170,11 @@ def _build_inprocess_demo(tmp_path):
 
 def test_c_program_links_against_the_library_and_fails_loudly_without_a_device(lib, tmp_path):
     """examples/inprocess_demo.c: the reference's call sites in C with libpgemb_b200.so where the reference links
-    hnswalg.o distfunc.o.  On a machine without a CUDA device it must refuse to run -- not compute on the CPU."""
+    hnswalg.o distfunc.o.  On a machine without a CUDA device it must refuse to run -- not compute on the CPU.  The demo is
+    started with CUDA_VISIBLE_DEVICES empty, so it sees no device on a machine with a GPU either."""
     import subprocess
-    if lib.pgemb_device_count() > 0:
-        pytest.skip("a CUDA device is present (the GPU variant of this test runs the demo)")
-    out = subprocess.run([_build_inprocess_demo(tmp_path)], capture_output=True, text=True, timeout=120)
+    out = subprocess.run([_build_inprocess_demo(tmp_path)], capture_output=True, text=True, timeout=120,
+                         env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
     assert out.returncode == 3 and "no CPU fallback" in out.stderr and out.stdout == ""
 
 

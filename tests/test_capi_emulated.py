@@ -440,7 +440,7 @@ def test_sharded_scan_two_shards(pg, oracle_mod, monkeypatch, metric, tc):
 
 def test_device_scan_edge_cases(pg, oracle_mod):
     import test_gpu_scan_umma as U
-    U.check_device_scan_edge_cases(pg, oracle_mod)
+    U.check_device_scan_edge_cases(pg, oracle_mod, device_memory=False)
 
 
 def test_ef_beyond_shared_memory(pg, G, oracle_mod, monkeypatch):

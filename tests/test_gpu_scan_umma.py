@@ -191,9 +191,10 @@ def test_scan_umma_default_policy(pg, monkeypatch):
         idx.close()
 
 
-def check_device_scan_edge_cases(pg, oracle_mod):
+def check_device_scan_edge_cases(pg, oracle_mod, device_memory=True):
     """pgemb_scan_topk_device on tables smaller than k, on an empty table and with every row deleted: counts, fill values
-    (~0 / +inf) and the host-pointer call's bytes."""
+    (~0 / +inf) and the host-pointer call's bytes.  device_memory=False for the host-emulated library, whose "device"
+    pointers are host pointers (a machine with a GPU runs that test too, so torch seeing a device does not decide it)."""
     from pg_embedding_b200 import _lib
     lib = _lib.load()
     rng = np.random.default_rng(3)
@@ -208,8 +209,8 @@ def check_device_scan_edge_cases(pg, oracle_mod):
                 labels |= np.uint64(1 << 48)
             idx.append(x, labels)
         ol = np.full((nq, k), 123, np.uint64); od = np.full((nq, k), 5.0, np.float32); on = np.full(nq, -1, np.int32)
-        import torch
-        if torch.cuda.is_available():      # a real device: the entry point takes device pointers
+        if device_memory:                  # a real device: the entry point takes device pointers
+            import torch
             tq = torch.from_numpy(q).cuda(); tl = torch.from_numpy(ol.view(np.int64)).cuda(); td = torch.from_numpy(od).cuda(); tn = torch.from_numpy(on).cuda()
             _lib.check(lib.pgemb_scan_topk_device(idx.dev, nq, tq.data_ptr(), k, tl.data_ptr(), td.data_ptr(), tn.data_ptr(), None))
             torch.cuda.synchronize()

@@ -445,14 +445,13 @@ def test_two_replicas_stay_identical_and_share_the_searches(emulated_lib, oracle
 
 
 def test_sidecar_refuses_to_start_without_a_device(tmp_path):
-    """No CPU fallback anywhere: with the product library and no CUDA device the sidecar exits instead of serving."""
+    """No CPU fallback anywhere: with the product library and no CUDA device the sidecar exits instead of serving.  The
+    sidecar is started with CUDA_VISIBLE_DEVICES empty, so it sees no device on a machine with a GPU either."""
     import subprocess
     from pg_embedding_b200 import build, sidecar
     build.build()
-    import pg_embedding_b200 as pg
-    if pg.device_count() > 0:
-        pytest.skip("a CUDA device is present")
-    res = subprocess.run([sidecar.SERVER_PATH, "--shm", f"/pgemb_test_nodev_{os.getpid()}"], capture_output=True, text=True, timeout=120)
+    res = subprocess.run([sidecar.SERVER_PATH, "--shm", f"/pgemb_test_nodev_{os.getpid()}"], capture_output=True, text=True, timeout=120,
+                         env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
     assert res.returncode == 4 and "no CPU fallback" in res.stderr
 
 
